@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the hot path: SS2D selective scan forward+backward, patch-tokens/s and % of the HBM roofline.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME] [--no-extras]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME] [--no-extras] [--dump-outputs DIR]
 
 The metric is quoted at two sequence lengths, so a STEP = one forward + one backward of the selective-scan op at BOTH of them:
 L = 196 (224 x 224 images, 14 x 14 tokens; B = 148 / GPU) and L = 6400 (1280 x 1280, 80 x 80 tokens; B = 16 / GPU), with SS2D's
@@ -119,6 +119,35 @@ def make_inputs(w, device, seed=0, dtype=torch.bfloat16):
     return dict(u=u, delta=delta, A=A.to(device), B=Bm, C=C, D=D.to(device), bias=bias.to(device), dout=dout, z=z)
 
 
+DUMP_MAX_ELEMS = 1 << 20       # per array; larger outputs are dumped as a fixed sample (4 MB in float32)
+DUMP_MAX_BYTES = 64 << 20      # all arrays of one dump together
+GRAD_NAMES = ("du", "ddelta", "dA", "dB", "dC", "dD", "ddelta_bias", "dz")
+
+
+def dump_outputs(path, names, results):
+    """Writes what the caller of each workload's fwd + bwd receives -- out, the last scan state and every gradient -- as
+    float32 `path/<workload>.<name>.npy`.  An array of more than DUMP_MAX_ELEMS elements is replaced by the elements at
+    DUMP_MAX_ELEMS sorted flat indices drawn with a seed-0 generator, so equal shapes are always sampled at the same places
+    and two builds can be compared array for array."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    arrays = {}
+    for wname, (out, x, grads) in zip(names, results):
+        named = [("out", out), ("last_state", x[:, :, -1, 1::2])] + list(zip(GRAD_NAMES, grads))
+        for name, t in named:
+            if t is None:
+                continue
+            flat = t.reshape(-1)
+            if flat.numel() > DUMP_MAX_ELEMS:
+                idx = torch.randint(flat.numel(), (DUMP_MAX_ELEMS,), generator=torch.Generator().manual_seed(0)).sort().values
+                t = flat[idx.to(flat.device)]
+            arrays[f"{wname}.{name}"] = t.float().cpu().numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_MAX_BYTES, f"output dump of {total} bytes exceeds {DUMP_MAX_BYTES}"
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 class ClockSampler:
     """SM clock / throttle reasons sampled DURING the timed region (B200_PROFILING.md): NVML polled every ~2 ms from a
     background thread (the timed region is only a few ms long, too short for `nvidia-smi -lms`)."""
@@ -174,15 +203,16 @@ class ClockSampler:
         return out
 
 
-def run_device_steps(inps, steps, warmup, dist_grads=None):
+def run_device_steps(inps, steps, warmup, dist_grads=None, last_outputs=None):
     """K timed steps on resident inputs; a step = fwd + bwd of every workload in `inps` (a list), then the gradient exchange.
-    Returns (total_ms, [fwd_ms_avg per workload], [bwd_ms_avg per workload])."""
+    Returns (total_ms, [fwd_ms_avg per workload], [bwd_ms_avg per workload]).  If `last_outputs` is a list, the results of
+    the last step are appended to it, one (out, x, grads) per workload."""
     from medical_image_analysis_b200 import scan_bwd, scan_fwd
     if isinstance(inps, dict):
         inps = [inps]
     nw = len(inps)
 
-    def one(ev=None, last=False):
+    def one(ev=None, last=False, keep=None):
         g = None
         for wi, inp in enumerate(inps):
             out_f32 = inp["dout"].dtype == torch.float32 and inp["u"].dtype != torch.float32
@@ -197,6 +227,8 @@ def run_device_steps(inps, steps, warmup, dist_grads=None):
                          out if z is not None else None, True, hblk=hblk)
             if ev:
                 ev[3 * wi + 2].record()
+            if keep is not None:
+                keep.append((out, x, g))
         if dist_grads is not None:
             dist_grads(g, last)
         if ev:
@@ -207,7 +239,7 @@ def run_device_steps(inps, steps, warmup, dist_grads=None):
     evs = [[torch.cuda.Event(enable_timing=True) for _ in range(3 * nw + 1)] for _ in range(steps)]
     torch.cuda.synchronize()
     for k in range(steps):
-        one(evs[k], k == steps - 1)
+        one(evs[k], k == steps - 1, last_outputs if k == steps - 1 else None)
     torch.cuda.synchronize()
     total = evs[0][0].elapsed_time(evs[-1][3 * nw])
     fwd = [sum(e[3 * wi].elapsed_time(e[3 * wi + 1]) for e in evs) / steps for wi in range(nw)]
@@ -518,7 +550,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-modules", action="store_true")
     ap.add_argument("--batch", type=int, default=0, help="override the per-GPU batch (single-workload runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<workload>.<name>.npy "
+                                                          "(float32, large arrays as a fixed sample; rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl b200)")
     names = list(HEADLINE) if args.workload == "headline" else [args.workload]
     ws = [dict(WORKLOADS[n]) for n in names]
     if args.batch > 0 and len(ws) == 1:
@@ -609,15 +647,22 @@ def main():
         dist.barrier()
     torch.cuda.synchronize()
     sampler.start()
-    run_device_steps(inps, max(3, args.warmup), 0, dist_grads)          # warm-up (>= 3 steps), also the sustained pre-roll
+    # a dump keeps the last step's outputs alive while the step still allocates; the warm-up keeps its last step's too, so
+    # that the memory this takes is already in the caching allocator and the timed step does not have to ask the driver
+    dump = rank == 0 and args.dump_outputs
+    run_device_steps(inps, max(3, args.warmup), 0, dist_grads, [] if dump else None)   # warm-up (>= 3 steps), also the sustained pre-roll
     time.sleep(0.02)
     sampler.mark()
     launches0 = _lib.launch_count()
     if world > 1:
         dist.barrier()
-    total_ms, fwd_ms, bwd_ms = run_device_steps(inps, args.steps, 0, dist_grads)
+    last_outputs = [] if dump else None
+    total_ms, fwd_ms, bwd_ms = run_device_steps(inps, args.steps, 0, dist_grads, last_outputs)
     launches = _lib.launch_count() - launches0
     clocks = sampler.stop()
+    if dump:
+        dump_outputs(args.dump_outputs, names, last_outputs)
+        del last_outputs
     total_ms = dp.max_over_ranks(total_ms, dev)
     value = sum(tokens) * world * args.steps / (total_ms * 1e-3)
 
