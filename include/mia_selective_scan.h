@@ -128,6 +128,12 @@ size_t mia_selective_scan_bwd_workspace(const mia_ss_params *p);
  * casts (:347) and delta-group folds (:348-353). */
 int mia_selective_scan_bwd(const mia_ss_params *p, void *cuda_stream);
 
+/* Which kernel mia_selective_scan_fwd (backward = 0) / _bwd (backward = 1) would launch for *p, and its geometry, as one
+ * line of space-separated key=value pairs starting with "kernel=". sms / smem_optin describe the device (<= 0: query the
+ * current device); when both are given no CUDA call is made. Tensor maps are not encoded (assumed encodable).
+ * Validates *p like the call itself (the backward's workspace included) and returns the same error codes. */
+int mia_ss_describe_plan(const mia_ss_params *p, int backward, int sms, int smem_optin, char *buf, size_t buf_len);
+
 /* CrossScan / CrossMerge of SS2D (R2GenCSR/VMamba/classification/models/vmamba.py:25-67, csm_triton.py:163-235).
  * x, y: (batch, channels, H, W) contiguous; xs, ys: (batch, 4, channels, H*W) contiguous; same dtype in and out.
  * scan: xs[:,0] = row-major, xs[:,1] = column-major, xs[:,2:4] = their reversals.  merge = its adjoint (fp32 sum).

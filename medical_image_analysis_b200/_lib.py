@@ -88,6 +88,9 @@ def lib() -> ctypes.CDLL:
         L.mia_ss_block_state_floats.restype = ctypes.c_size_t
         L.mia_ss_fwd_writes_block_states.argtypes = [ctypes.POINTER(MiaSSParams)]
         L.mia_ss_fwd_writes_block_states.restype = ctypes.c_int
+        L.mia_ss_describe_plan.argtypes = [ctypes.POINTER(MiaSSParams), ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_char_p,
+                                           ctypes.c_size_t]
+        L.mia_ss_describe_plan.restype = ctypes.c_int
         if L.mia_abi_version() != 2:
             raise RuntimeError(f"libmia_scan.so ABI version {L.mia_abi_version()} != 2: rebuild it")
         _lib = L

@@ -1,36 +1,22 @@
 // Host side of libmia_scan.so: argument validation (the reference's TORCH_CHECKs,
-// selective_scan_oflex.cpp:152-204 / 245-312), tile planning, launches, the finalize kernel that folds the
-// backward's deterministic partials, and the extern "C" surface declared in include/mia_selective_scan.h.
+// selective_scan_oflex.cpp:152-204 / 245-312), the planner that picks a kernel family and its geometry for a call
+// (plan_fwd / plan_bwd, also behind mia_ss_describe_plan and mia_ss_fwd_writes_block_states), one launch per direction,
+// the finalize kernel that folds the backward's deterministic partials, and the extern "C" surface declared in
+// include/mia_selective_scan.h.  The kernels are reached only through the launchers declared in scan_args.h and
+// instantiated in the per-dtype scan_{fwd,bwd}_*.cu files: this file compiles none of them.
 #include <algorithm>
 #include <atomic>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <initializer_list>
+#include <type_traits>
 
 #include "../../include/mia_selective_scan.h"
+#include "scan_args.h"
 #include "scan_common.cuh"
-#include "scan_bwd_rows.cuh"
-#include "scan_bwd_rowsn.cuh"
-#include "scan_bwd_cw.cuh"
 #include "tma_host.h"
-#include "scan_fwd_rowsn.cuh"
-#include "scan_fwd_stream.cuh"
-#include "scan_fwd_chunks.cuh"
-#include "scan_fwd_cw.cuh"
-
-namespace mia {
-template <typename T> cudaError_t launch_fwd_rows(const RowsArgs &, int, bool, cudaStream_t);
-template <typename T> cudaError_t launch_fwd_rowsn(const RowsNArgs &, int, bool, cudaStream_t);
-template <typename T> cudaError_t launch_fwd_stream(const StreamArgs &, int, bool, cudaStream_t);
-template <typename T> cudaError_t launch_fwd_chunks(const ChunkArgs &, int, bool, cudaStream_t);
-template <typename T> cudaError_t launch_fwd_cw(const CUtensorMap *, const CwFwdArgs &, int, bool, cudaStream_t);
-template <typename T> cudaError_t launch_bwd_rows(const RowsBwdArgs &, int, bool, cudaStream_t);
-template <typename T> cudaError_t launch_bwd_rowsn(const RowsNBwdArgs &, int, bool, cudaStream_t);
-template <typename T> cudaError_t launch_bwd_cw(const CUtensorMap *, const CwBwdArgs &, int, bool, cudaStream_t);
-template <typename T> cudaError_t launch_fwd_any(const ScanArgs &, int, cudaStream_t);
-template <typename T> cudaError_t launch_bwd_any(const ScanArgs &, int, cudaStream_t);
-}  // namespace mia
 
 namespace {
 
@@ -198,7 +184,7 @@ int validate_common(const mia_ss_params &p) {
     return MIA_OK;
 }
 
-void fill_common(mia::ScanArgs &a, const mia_ss_params &p, const Plan &pl, bool bwd) {
+void fill_common(mia::ScanArgs &a, const mia_ss_params &p, const Plan &pl) {
     memset(&a, 0, sizeof(a));
     a.batch = p.batch; a.dim = p.dim; a.L = p.seqlen; a.N = p.dstate; a.G = p.n_groups; a.delta_dim = p.delta_dim;
     a.rows_per_group = p.dim / p.n_groups;
@@ -218,7 +204,6 @@ void fill_common(mia::ScanArgs &a, const mia_ss_params &p, const Plan &pl, bool 
     a.flat_z = a.has_z && whole && p.z_d_stride == p.seqlen;
     a.flat_B = whole && p.B_dstate_stride == p.seqlen;
     a.flat_C = whole && p.C_dstate_stride == p.seqlen;
-    (void)bwd;
 }
 
 // Shared-memory carve-up.  Returns false if not even two row stages fit.
@@ -249,8 +234,7 @@ bool layout_smem(mia::ScanArgs &a, int es, int eso, bool bwd, int smem_max) {
     const int bars = round_up((2 * mia::kMaxStages + 2 * mia::kGroupStages) * 8, 128);
     const int carry = round_up(bwd ? (2 * a.RS * a.N + 2 * a.RS) * 4 : a.RS * a.N * 8, 128);
     const int red = bwd ? a.n_consumer_warps * 256 * 4 : 0;
-    const int bcf = 0;   // (an fp32 copy of the B / C chunk for the d_state > 1 fast backward was tried and removed)
-    const int fixed = mia::kGroupStages * a.gstage_bytes + bars + carry + red + bcf;
+    const int fixed = mia::kGroupStages * a.gstage_bytes + bars + carry + red;
     int stages = (smem_max - fixed) / a.stage_bytes;
     if (stages > mia::kMaxStages) stages = mia::kMaxStages;
     if (stages < 2) return false;
@@ -259,8 +243,7 @@ bool layout_smem(mia::ScanArgs &a, int es, int eso, bool bwd, int smem_max) {
     a.off_bars = a.off_groups + mia::kGroupStages * a.gstage_bytes;
     a.off_carry = a.off_bars + bars;
     a.off_red = a.off_carry + carry;
-    a.off_bcf = bcf ? a.off_red + red : 0;
-    a.smem_bytes = a.off_red + red + bcf;
+    a.smem_bytes = a.off_red + red;
     return true;
 }
 
@@ -271,7 +254,7 @@ int plan_and_layout(const mia_ss_params &p, const DeviceInfo &di, bool bwd, Plan
     const int es = esize(p.itype), eso = esize(p.otype);
     const int rpg = p.dim / p.n_groups;
     for (;;) {
-        fill_common(a, p, pl, bwd);
+        fill_common(a, p, pl);
         if (bwd) {
             const bool whole = pl.n_chunks == 1;
             a.flat_dout = whole && p.dout_d_stride == p.seqlen;
@@ -288,6 +271,49 @@ int plan_and_layout(const mia_ss_params &p, const DeviceInfo &di, bool bwd, Plan
     }
 }
 
+// ---- Eligibility rules and argument-block pieces shared by the kernel families
+// (batch stride, row stride) pairs of (batch, rows, L) tensors: every row L contiguous tokens, rows back to back
+bool dense_rows(const mia_ss_params &p, std::initializer_list<std::pair<long long, long long>> tensors) {
+    for (const auto &t : tensors)
+        if (t.second != p.seqlen || t.first != (long long)p.dim * p.seqlen) return false;
+    return true;
+}
+bool fwd_rows_dense(const mia_ss_params &p) {          // u, delta, out
+    return dense_rows(p, {{p.u_batch_stride, p.u_d_stride}, {p.delta_batch_stride, p.delta_d_stride}, {p.out_batch_stride, p.out_d_stride}});
+}
+bool bwd_rows_dense(const mia_ss_params &p) {          // u, delta, dout, du, ddelta
+    return dense_rows(p, {{p.u_batch_stride, p.u_d_stride}, {p.delta_batch_stride, p.delta_d_stride}, {p.dout_batch_stride, p.dout_d_stride},
+                          {p.du_batch_stride, p.du_d_stride}, {p.ddelta_batch_stride, p.ddelta_d_stride}});
+}
+bool aligned16(std::initializer_list<const void *> ptrs) {
+    uintptr_t bits = 0;
+    for (const void *q : ptrs) bits |= (uintptr_t)q;
+    return (bits & 15) == 0;
+}
+// The d_state 1 kernels read A as one value per row.
+bool a_per_row(const mia_ss_params &p) { return p.A_d_stride == 1 || p.dim == 1; }
+// Preconditions of every d_state 1 kernel that gives a lane one row: no z gate, delta per row, whole 32-row batches of one
+// group, rows of whole 4-token pieces.
+bool lane_per_row(const mia_ss_params &p) {
+    return p.dstate == 1 && !p.z && p.delta_dim == p.dim && (p.dim / p.n_groups) % 32 == 0 && p.seqlen % 4 == 0;
+}
+
+// Fields every row-serial / column-walk argument block has; the rest of the block starts zeroed.
+template <typename R>
+void init_args(R &r, const mia_ss_params &p) {
+    memset(&r, 0, sizeof(r));
+    r.batch = p.batch; r.dim = p.dim; r.L = p.seqlen; r.G = p.n_groups; r.rows_per_group = p.dim / p.n_groups;
+    r.softplus = p.delta_softplus;
+    r.A = p.A; r.B = p.B; r.C = p.C; r.D = p.D; r.delta_bias = p.delta_bias;
+    r.B_bs = p.B_batch_stride; r.B_gs = p.B_group_stride; r.C_bs = p.C_batch_stride; r.C_gs = p.C_group_stride;
+}
+
+// Resident CTAs per SM for a kernel of `smem` bytes of dynamic shared memory (1 KB reserved per CTA), at most `cap`.
+int resident_ctas(int smem, int cap) {
+    const int n = (227 * 1024) / (smem + 1024);
+    return n > cap ? cap : n;
+}
+
 // Geometry of the column-walk kernels (scan_fwd_cw.cuh / scan_bwd_cw.cuh): g rows per tensor-map row.  A pure function of the
 // problem's sizes and dtypes (and the SM count) -- it also fixes the LAYOUT of the block states (hblk), which forward and backward must agree on.
 // A tensor-map row must be a multiple of 16 bytes (else the map cannot be encoded); it SHOULD be a multiple of 32 (else every
@@ -298,9 +324,9 @@ int plan_and_layout(const mia_ss_params &p, const DeviceInfo &di, bool bwd, Plan
 // lane).  fp32 rows (L % 4 == 0) are always legal: g = 1.
 bool cw_geometry(const mia_ss_params &p, int sms, int &g) {
     const int es = esize(p.itype), L = p.seqlen;
-    if (p.dstate != 1 || p.z || p.delta_dim != p.dim || (L % 4) || p.n_groups < 1) return false;
+    if (!lane_per_row(p)) return false;
     const int rpg = p.dim / p.n_groups;
-    if (es == 4) { g = 1; return rpg % 32 == 0; }
+    if (es == 4) { g = 1; return true; }
     const int want = (L % 16 == 0) ? 1 : (L % 8 == 0) ? 2 : 4;
     // Items are 32 g rows: a larger g halves their number, and a problem that fills the resident slots a little more than once
     // pays a whole second round (measured, gpurun r2fin2, B = 64, L = 196, fp32 out: 1536 items on 1332 - 1480 slots, forward
@@ -321,27 +347,23 @@ bool cw_geometry(const mia_ss_params &p, int sms, int &g) {
     return false;
 }
 
-// Row-serial forward (scan_fwd_rows.cuh): eligibility + argument block.  Returns false when the warp-scan kernels must run.
+// ---- One planner per kernel family: eligibility + argument block + grid.  Each returns false when the shape is not one its
+// kernel takes (the caller then tries the next family).
+
+// Row-serial forward (scan_fwd_rows.cuh).
 bool plan_rows_fwd(const mia_ss_params &p, const DeviceInfo &di, mia::RowsArgs &r, int &grid) {
     const int es = esize(p.itype), L = p.seqlen;
-    const int rpg = p.dim / p.n_groups;
-    if (p.dstate != 1 || p.z || p.delta_dim != p.dim || (rpg % 32) || (L % 4)) return false;
-    if (dbg_knob("MIA_NO_ROWS_FWD")) return false;
-    auto dense = [&](long long bs, long long ds) { return ds == L && bs == (long long)p.dim * L; };
-    if (!dense(p.u_batch_stride, p.u_d_stride) || !dense(p.delta_batch_stride, p.delta_d_stride) ||
-        !dense(p.out_batch_stride, p.out_d_stride)) return false;
-    if (p.A_d_stride != 1 && p.dim > 1) return false;
-    if (((uintptr_t)p.u | (uintptr_t)p.delta | (uintptr_t)p.out) & 15) return false;
-    memset(&r, 0, sizeof(r));
+    if (!lane_per_row(p) || dbg_knob("MIA_NO_ROWS_FWD")) return false;
+    if (!fwd_rows_dense(p) || !a_per_row(p) || !aligned16({p.u, p.delta, p.out})) return false;
+    init_args(r, p);
     const int budget = 13 * 1024;                               // bytes of one [32 x chunk] tile (8 warps per SM at 2-byte dtypes)
     int Lc = L;
     if (32 * L * es > budget) {
         if ((L * es) % 16) return false;                        // per-row pieces must start 16-byte aligned
         Lc = budget / (32 * es) / 8 * 8;
     }
-    r.batch = p.batch; r.dim = p.dim; r.L = L; r.G = p.n_groups; r.rows_per_group = rpg; r.softplus = p.delta_softplus;
     r.Lc = Lc; r.n_lchunks = (L + Lc - 1) / Lc;
-    r.n_items = p.batch * p.n_groups * (rpg / 32);
+    r.n_items = p.batch * p.n_groups * (r.rows_per_group / 32);
     r.tile_bytes = round_up(32 * Lc * es, 128);
     r.bc_bytes = 0;
     r.off_bc32 = 2 * r.tile_bytes;
@@ -349,34 +371,27 @@ bool plan_rows_fwd(const mia_ss_params &p, const DeviceInfo &di, mia::RowsArgs &
     r.smem_bytes = r.stage_bytes + 128;
     if (r.smem_bytes > di.smem_optin) return false;
     r.xchunks = mia_ss_num_chunks(L); r.xchunk_tokens = mia_ss_chunk_len(L);
-    r.u = p.u; r.delta = p.delta; r.A = p.A; r.B = p.B; r.C = p.C; r.D = p.D; r.delta_bias = p.delta_bias; r.out = p.out; r.x = p.x;
-    r.B_bs = p.B_batch_stride; r.B_gs = p.B_group_stride; r.C_bs = p.C_batch_stride; r.C_gs = p.C_group_stride;
-    const int per_sm = di.smem_optin / (r.smem_bytes + 1024) > 0 ? (227 * 1024) / (r.smem_bytes + 1024) : 1;
-    grid = di.sms * (per_sm < 1 ? 1 : (per_sm > 8 ? 8 : per_sm));
+    r.u = p.u; r.delta = p.delta; r.out = p.out; r.x = p.x;
+    const int per_sm = di.smem_optin / (r.smem_bytes + 1024) > 0 ? resident_ctas(r.smem_bytes, 8) : 1;
+    grid = di.sms * (per_sm < 1 ? 1 : per_sm);
     if (grid > r.n_items) grid = r.n_items;
     return true;
 }
 
-// Column-walk forward (scan_fwd_cw.cuh): eligibility, argument block, tensor maps (u, delta, out).
+// Column-walk forward (scan_fwd_cw.cuh): eligibility, argument block, tensor maps (u, delta, out; not encoded when tm is null).
 bool plan_cw_fwd(const mia_ss_params &p, const DeviceInfo &di, mia::CwFwdArgs &r, CUtensorMap *tm, int &grid) {
     const int es = esize(p.itype), eo = esize(p.otype), L = p.seqlen;
     int g = 0;
-    if (!cw_geometry(p, di.sms, g)) return false;
-    if (dbg_knob("MIA_NO_CW_FWD")) return false;
+    if (!cw_geometry(p, di.sms, g) || dbg_knob("MIA_NO_CW_FWD")) return false;
+    if (!fwd_rows_dense(p) || !a_per_row(p) || !aligned16({p.u, p.delta, p.out})) return false;
     const int rpg = p.dim / p.n_groups;
-    auto dense = [&](long long bs, long long ds) { return ds == L && bs == (long long)p.dim * L; };
-    if (!dense(p.u_batch_stride, p.u_d_stride) || !dense(p.delta_batch_stride, p.delta_d_stride) ||
-        !dense(p.out_batch_stride, p.out_d_stride)) return false;
-    if (p.A_d_stride != 1 && p.dim > 1) return false;
-    if (((uintptr_t)p.u | (uintptr_t)p.delta | (uintptr_t)p.out) & 15) return false;
     const unsigned long long trows = (unsigned long long)p.batch * p.dim / g, tcols = (unsigned long long)g * L;
     if (tcols >= (1ull << 31) || trows >= (1ull << 31)) return false;
     const int n_items = p.batch * p.n_groups * (rpg / (32 * g));
     // few long rows: the chunk-parallel kernel (scan_fwd_chunks.cuh) has more warps to offer than one per 32 rows
     if (n_items < 4 * di.sms && (L + mia::kChunkTok - 1) / mia::kChunkTok >= 2 && !dbg_knob("MIA_FORCE_CW_FWD")) return false;
-    memset(&r, 0, sizeof(r));
+    init_args(r, p);
     r.zero = 0;                                                  // (the kernel XORs parameter loads with it: scan_fwd_cw.cuh, settle)
-    r.batch = p.batch; r.dim = p.dim; r.L = L; r.G = p.n_groups; r.rows_per_group = rpg; r.softplus = p.delta_softplus;
     r.g = g; r.n_items = n_items;
     r.nwin = (g * L + mia::kCwTok - 1) / mia::kCwTok;
     r.ngrp = (g * L + 15) / 16;
@@ -384,17 +399,16 @@ bool plan_cw_fwd(const mia_ss_params &p, const DeviceInfo &di, mia::CwFwdArgs &r
     const int tile_i = 32 * mia::kCwTok * es, tile_o = 32 * mia::kCwTok * eo;
     r.stage_bytes = 2 * tile_i;
     // stages: 4 unless 3 gives a better-balanced last round (more resident warps)
-    int best_ns = 0, best_per_sm = 0;
+    int best_ns = 0;
     double best_eff = -1.0;
     for (int ns = 4; ns >= 3; --ns) {
         const int smem = ns * r.stage_bytes + (of32 ? 2 * tile_o : 0) + 2 * mia::kCwTok * 4 + 8 * ns + 16;
-        int per_sm = (227 * 1024) / (smem + 1024);
-        if (per_sm > 16) per_sm = 16;
+        const int per_sm = resident_ctas(smem, 16);
         if (per_sm < 1) continue;
         const long long slots = (long long)di.sms * per_sm;
         const long long rounds = (n_items + slots - 1) / slots;
         const double eff = (double)n_items / (double)(rounds * slots) * (per_sm >= 8 ? 1.0 : per_sm / 8.0);
-        if (eff > best_eff + 0.03) { best_eff = eff; best_ns = ns; best_per_sm = per_sm; }
+        if (eff > best_eff + 0.03) { best_eff = eff; best_ns = ns; }
     }
     if (!best_ns) return false;
     r.ns = dbg_int("MIA_CW_STAGES", best_ns);
@@ -403,106 +417,82 @@ bool plan_cw_fwd(const mia_ss_params &p, const DeviceInfo &di, mia::CwFwdArgs &r
     r.off_bar = r.off_bc32 + 2 * mia::kCwTok * 4;
     r.smem_bytes = r.off_bar + 8 * r.ns + 16;
     r.xchunks = mia_ss_num_chunks(L); r.xchunk_tokens = mia_ss_chunk_len(L);
-    r.A = p.A; r.B = p.B; r.C = p.C; r.D = p.D; r.delta_bias = p.delta_bias; r.x = p.x; r.hblk = p.hblk;
-    r.B_bs = p.B_batch_stride; r.B_gs = p.B_group_stride; r.C_bs = p.C_batch_stride; r.C_gs = p.C_group_stride;
+    r.x = p.x; r.hblk = p.hblk;
     const void *ptrs[3] = {p.u, p.delta, p.out};
-    for (int i = 0; i < 3; ++i) {
+    for (int i = 0; tm && i < 3; ++i) {
         const int e = i == 2 ? eo : es;
         const int trc = mia::tma_make_2d(&tm[i], ptrs[i], trows, tcols, tcols * e, 32, mia::kCwTok, e, mia::kCwTok * e);
         if (trc != 0) { MIA_TRACE("cw fwd: tensor map %d rejected (CUresult %d)", i, trc); return false; }
     }
-    int per_sm = (227 * 1024) / (r.smem_bytes + 1024);
-    if (per_sm > 16) per_sm = 16;
+    int per_sm = resident_ctas(r.smem_bytes, 16);
     per_sm = std::min(per_sm, dbg_int("MIA_CW_MAXPERSM", per_sm));
     if (per_sm < 1) return false;
     const long long slots = (long long)di.sms * per_sm;
     const long long rounds = (n_items + slots - 1) / slots;
     grid = (int)((n_items + rounds - 1) / rounds);              // equal rounds per CTA
-    (void)best_per_sm;
     return true;
 }
 
-// Chunk-parallel forward for long rows and few 32-row batches (scan_fwd_chunks.cuh): eligibility + argument block.
+// Chunk-parallel forward for long rows and few 32-row batches (scan_fwd_chunks.cuh).
 bool plan_chunks_fwd(const mia_ss_params &p, const DeviceInfo &di, mia::ChunkArgs &r, int &grid) {
     const int es = esize(p.itype), eo = esize(p.otype), L = p.seqlen;
-    const int rpg = p.dim / p.n_groups;
-    if (p.dstate != 1 || p.z || p.delta_dim != p.dim || (rpg % 32) || (L % 4)) return false;
-    if (dbg_knob("MIA_NO_ROWS_FWD") || dbg_knob("MIA_NO_CHUNKS_FWD")) return false;
+    if (!lane_per_row(p) || dbg_knob("MIA_NO_ROWS_FWD") || dbg_knob("MIA_NO_CHUNKS_FWD")) return false;
     const int nch = (L + mia::kChunkTok - 1) / mia::kChunkTok;
     if (nch < 2 || mia_ss_chunk_len(L) != mia::kChunkTok || ((L * es) % 16) || ((L * eo) % 16)) return false;
-    const int n_batches = p.batch * p.n_groups * (rpg / 32);
+    const int n_batches = p.batch * p.n_groups * (p.dim / p.n_groups / 32);
     if (n_batches >= 4 * di.sms) return false;                 // enough rows: the serial row walk fills the machine
-    auto dense = [&](long long bs, long long ds) { return ds == L && bs == (long long)p.dim * L; };
-    if (!dense(p.u_batch_stride, p.u_d_stride) || !dense(p.delta_batch_stride, p.delta_d_stride) ||
-        !dense(p.out_batch_stride, p.out_d_stride)) return false;
-    if (p.A_d_stride != 1 && p.dim > 1) return false;
-    if (((uintptr_t)p.u | (uintptr_t)p.delta | (uintptr_t)p.out) & 15) return false;
-    memset(&r, 0, sizeof(r));
-    r.batch = p.batch; r.dim = p.dim; r.L = L; r.G = p.n_groups; r.rows_per_group = rpg; r.softplus = p.delta_softplus;
+    if (!fwd_rows_dense(p) || !a_per_row(p) || !aligned16({p.u, p.delta, p.out})) return false;
+    init_args(r, p);
     r.n_chunks = nch;
     r.n_items = n_batches * nch;
     r.tile_bytes = round_up(32 * (mia::kChunkTok * es + 16), 128);
     r.off_bc32 = 2 * r.tile_bytes;
     r.off_bar = r.off_bc32 + 2 * mia::kChunkTok * 4;
     r.smem_bytes = r.off_bar + 128;
-    int per_sm = (227 * 1024) / (r.smem_bytes + 1024);
+    const int per_sm = resident_ctas(r.smem_bytes, 8);
     if (per_sm < 3) return false;
-    if (per_sm > 8) per_sm = 8;
-    r.u = p.u; r.delta = p.delta; r.A = p.A; r.B = p.B; r.C = p.C; r.D = p.D; r.delta_bias = p.delta_bias; r.out = p.out; r.x = p.x;
-    r.B_bs = p.B_batch_stride; r.B_gs = p.B_group_stride; r.C_bs = p.C_batch_stride; r.C_gs = p.C_group_stride;
+    r.u = p.u; r.delta = p.delta; r.out = p.out; r.x = p.x;
     grid = di.sms * per_sm;
     if (grid > r.n_items) grid = r.n_items;
     return true;
 }
 
-// Streaming row-serial forward (scan_fwd_stream.cuh): eligibility + argument block.
+// Streaming row-serial forward (scan_fwd_stream.cuh).
 bool plan_stream_fwd(const mia_ss_params &p, const DeviceInfo &di, mia::StreamArgs &r, int &grid) {
     const int es = esize(p.itype), eo = esize(p.otype), L = p.seqlen;
-    const int rpg = p.dim / p.n_groups;
-    if (p.dstate != 1 || p.z || p.delta_dim != p.dim || (rpg % 32) || (L % 4)) return false;
-    if (dbg_knob("MIA_NO_ROWS_FWD") || dbg_knob("MIA_NO_STREAM_FWD")) return false;
-    auto dense = [&](long long bs, long long ds) { return ds == L && bs == (long long)p.dim * L; };
-    if (!dense(p.u_batch_stride, p.u_d_stride) || !dense(p.delta_batch_stride, p.delta_d_stride) ||
-        !dense(p.out_batch_stride, p.out_d_stride)) return false;
-    if (p.A_d_stride != 1 && p.dim > 1) return false;
+    if (!lane_per_row(p) || dbg_knob("MIA_NO_ROWS_FWD") || dbg_knob("MIA_NO_STREAM_FWD")) return false;
+    if (!fwd_rows_dense(p) || !a_per_row(p)) return false;
     const uintptr_t piece = 4 * es - 1, pieceo = 4 * eo - 1;    // every row start is a multiple of one 4-token piece
     if ((((uintptr_t)p.u | (uintptr_t)p.delta) & piece) || ((uintptr_t)p.out & pieceo)) return false;
     if (L > 256 && mia_ss_chunk_len(L) != 256) return false;
-    memset(&r, 0, sizeof(r));
-    r.batch = p.batch; r.dim = p.dim; r.L = L; r.G = p.n_groups; r.rows_per_group = rpg; r.softplus = p.delta_softplus;
-    r.n_items = p.batch * p.n_groups * (rpg / 32);
+    init_args(r, p);
+    r.n_items = p.batch * p.n_groups * (r.rows_per_group / 32);
     r.Lp = (L + 3) & ~3;
     const int pitch = mia::kStreamTok * es + 4 * es;
     r.off_bc32 = round_up(2 * 2 * 32 * pitch, 128);             // 2 stages x (u, delta)
     r.smem_bytes = r.off_bc32 + round_up(2 * r.Lp * 4, 128);
     if (r.smem_bytes > di.smem_optin) return false;
     r.xchunks = mia_ss_num_chunks(L);
-    r.u = p.u; r.delta = p.delta; r.A = p.A; r.B = p.B; r.C = p.C; r.D = p.D; r.delta_bias = p.delta_bias; r.out = p.out; r.x = p.x;
-    r.B_bs = p.B_batch_stride; r.B_gs = p.B_group_stride; r.C_bs = p.C_batch_stride; r.C_gs = p.C_group_stride;
-    int per_sm = (227 * 1024) / (r.smem_bytes + 1024);
-    if (per_sm > 16) per_sm = 16;                               // 128 registers per thread
+    r.u = p.u; r.delta = p.delta; r.out = p.out; r.x = p.x;
+    const int per_sm = resident_ctas(r.smem_bytes, 16);         // 128 registers per thread
     if (per_sm < 4) return false;
     grid = di.sms * per_sm;
     if (grid > r.n_items) grid = r.n_items;
     return true;
 }
 
-// Row-serial forward for d_state > 1 (scan_fwd_rowsn.cuh): eligibility + argument block.
+// Row-serial forward for d_state 8 / 16 (scan_fwd_rowsn.cuh).
 bool plan_rowsn_fwd(const mia_ss_params &p, const DeviceInfo &di, mia::RowsNArgs &r, int &grid) {
     const int es = esize(p.itype), L = p.seqlen, N = p.dstate;
     const int rpg = p.dim / p.n_groups;
-    if ((N != 16 && N != 8) || p.delta_dim != p.dim || (rpg % 32)) return false;
-    if (dbg_knob("MIA_NO_ROWS_FWD")) return false;
+    if ((N != 16 && N != 8) || p.delta_dim != p.dim || (rpg % 32) || dbg_knob("MIA_NO_ROWS_FWD")) return false;
     if (mia_ss_num_chunks(L) != 1) return false;                // whole rows, one checkpoint
-    auto dense = [&](long long bs, long long ds) { return ds == L && bs == (long long)p.dim * L; };
-    if (!dense(p.u_batch_stride, p.u_d_stride) || !dense(p.delta_batch_stride, p.delta_d_stride) ||
-        !dense(p.out_batch_stride, p.out_d_stride)) return false;
-    if (((uintptr_t)p.u | (uintptr_t)p.delta | (uintptr_t)p.out) & 15) return false;
-    if (p.z && (!dense(p.z_batch_stride, p.z_d_stride) || !dense(p.out_z_batch_stride, p.out_z_d_stride) ||
-                (((uintptr_t)p.z | (uintptr_t)p.out_z) & 15))) return false;
+    if (!fwd_rows_dense(p) || !aligned16({p.u, p.delta, p.out})) return false;
+    if (p.z && (!dense_rows(p, {{p.z_batch_stride, p.z_d_stride}, {p.out_z_batch_stride, p.out_z_d_stride}}) || !aligned16({p.z, p.out_z})))
+        return false;
     if ((32 * L * es) % 16) return false;
-    memset(&r, 0, sizeof(r));
-    r.batch = p.batch; r.dim = p.dim; r.L = L; r.G = p.n_groups; r.rows_per_group = rpg; r.N = N; r.softplus = p.delta_softplus;
+    init_args(r, p);
+    r.N = N;
     r.warps = p.z ? 2 : mia::kRowsNWarps;
     r.tiles_per_warp = p.z ? 3 : 2;
     const int W = r.warps;
@@ -514,34 +504,23 @@ bool plan_rowsn_fwd(const mia_ss_params &p, const DeviceInfo &di, mia::RowsNArgs
     r.smem_bytes = r.off_bar + 128;
     const int per_sm = (int)(233472 / (r.smem_bytes + 1024));
     if (per_sm < 1 || r.smem_bytes > di.smem_optin) return false;
-    r.u = p.u; r.delta = p.delta; r.A = p.A; r.B = p.B; r.C = p.C; r.D = p.D; r.delta_bias = p.delta_bias; r.out = p.out; r.x = p.x;
-    r.z = p.z; r.out_z = p.out_z;
-    r.A_ds = p.A_d_stride; r.A_ns = p.A_dstate_stride;
-    r.B_bs = p.B_batch_stride; r.B_gs = p.B_group_stride; r.B_ns = p.B_dstate_stride;
-    r.C_bs = p.C_batch_stride; r.C_gs = p.C_group_stride; r.C_ns = p.C_dstate_stride;
+    r.u = p.u; r.delta = p.delta; r.out = p.out; r.x = p.x; r.z = p.z; r.out_z = p.out_z;
+    r.A_ds = p.A_d_stride; r.A_ns = p.A_dstate_stride; r.B_ns = p.B_dstate_stride; r.C_ns = p.C_dstate_stride;
     grid = di.sms * (per_sm > 4 ? 4 : per_sm);
     if (grid > r.n_units) grid = r.n_units;
     return true;
 }
 
-// Row-serial backward (scan_bwd_rows.cuh): eligibility + argument block.  Returns false when the warp-scan kernels must run.
+// Row-serial backward (scan_bwd_rows.cuh).
 bool plan_rows_bwd(const mia_ss_params &p, const DeviceInfo &di, mia::RowsBwdArgs &r, int &grid) {
     const int es = esize(p.itype), eo = esize(p.otype), L = p.seqlen;
-    const int rpg = p.dim / p.n_groups;
-    if (p.dstate != 1 || p.z || p.delta_dim != p.dim || (rpg % 32) || (L % 4)) return false;
-    if (dbg_knob("MIA_NO_ROWS_BWD")) return false;
+    if (!lane_per_row(p) || dbg_knob("MIA_NO_ROWS_BWD")) return false;
     const int CH = mia::kRowsChunk;
     const int nch = (L + CH - 1) / CH;
     // long rows: x must hold a checkpoint every 256 tokens, and the per-row pieces of a tile must be 16-byte aligned
     if (nch > 1 && (mia_ss_chunk_len(L) != CH || !p.x || ((L * es) % 16) || ((L * eo) % 16))) return false;
-    auto dense = [&](long long bs, long long ds) { return ds == L && bs == (long long)p.dim * L; };
-    if (!dense(p.u_batch_stride, p.u_d_stride) || !dense(p.delta_batch_stride, p.delta_d_stride) ||
-        !dense(p.dout_batch_stride, p.dout_d_stride) || !dense(p.du_batch_stride, p.du_d_stride) ||
-        !dense(p.ddelta_batch_stride, p.ddelta_d_stride)) return false;
-    if (p.A_d_stride != 1 && p.dim > 1) return false;
-    if (((uintptr_t)p.u | (uintptr_t)p.delta | (uintptr_t)p.dout | (uintptr_t)p.du | (uintptr_t)p.ddelta) & 15) return false;
-    memset(&r, 0, sizeof(r));
-    r.batch = p.batch; r.dim = p.dim; r.L = L; r.G = p.n_groups; r.rows_per_group = rpg; r.softplus = p.delta_softplus;
+    if (!bwd_rows_dense(p) || !a_per_row(p) || !aligned16({p.u, p.delta, p.dout, p.du, p.ddelta})) return false;
+    init_args(r, p);
     r.n_chunks = nch;
     const int span = nch == 1 ? L : CH;                         // tokens of a row resident at a time
     r.t0_pct = dbg_int("MIA_T0_PCT", 52);   // share of a chunk for the half that has no Gs to accumulate
@@ -549,7 +528,7 @@ bool plan_rows_bwd(const mia_ss_params &p, const DeviceInfo &di, mia::RowsBwdArg
     const int longer = T0 > span - T0 ? T0 : span - T0;
     r.nblk = (longer + mia::kBlk - 1) / mia::kBlk;
     r.Lp = (span + mia::kBlk - 1) / mia::kBlk * mia::kBlk + mia::kBlk;
-    r.n_items = p.batch * p.n_groups * (rpg / 32);
+    r.n_items = p.batch * p.n_groups * (r.rows_per_group / 32);
     r.tile_bytes = round_up(32 * (span * es + (nch > 1 ? 16 : 0)), 128);
     r.tileo_bytes = round_up(32 * (span * eo + (nch > 1 ? 16 : 0)), 128);
     r.off_delta = r.tile_bytes;
@@ -559,12 +538,9 @@ bool plan_rows_bwd(const mia_ss_params &p, const DeviceInfo &di, mia::RowsBwdArg
     r.off_xch = r.off_ck + 3 * r.nblk * 128;                    // ck of both halves + ckm
     r.off_bar = r.off_xch + 7 * 128;
     r.smem_bytes = r.off_bar + 128;
-    int per_sm = (227 * 1024) / (r.smem_bytes + 1024);
+    const int per_sm = resident_ctas(r.smem_bytes, 5);          // 64 threads x 168 registers: 3 warps per scheduler
     if (per_sm < 3) return false;                               // too few resident warps to hide the dependent chains
-    if (per_sm > 5) per_sm = 5;                                 // 64 threads x 168 registers: 3 warps per scheduler
-    r.u = p.u; r.delta = p.delta; r.A = p.A; r.B = p.B; r.C = p.C; r.D = p.D; r.delta_bias = p.delta_bias; r.dout = p.dout;
-    r.du = p.du; r.ddelta = p.ddelta; r.x = p.x;
-    r.B_bs = p.B_batch_stride; r.B_gs = p.B_group_stride; r.C_bs = p.C_batch_stride; r.C_gs = p.C_group_stride;
+    r.u = p.u; r.delta = p.delta; r.dout = p.dout; r.du = p.du; r.ddelta = p.ddelta; r.x = p.x;
     grid = di.sms * per_sm;
     // Long rows: a CTA walks its 32 rows chunk by chunk and each chunk is latency-bound (load -> phase 1 -> exchange ->
     // phase 2 -> store), so this path only wins while every item gets its own resident CTA (measured on B200, L = 6400:
@@ -574,25 +550,24 @@ bool plan_rows_bwd(const mia_ss_params &p, const DeviceInfo &di, mia::RowsBwdArg
     return true;
 }
 
-// Column-walk backward (scan_bwd_cw.cuh): eligibility, argument block, tensor maps (u, delta, dout, du, ddelta).
+// Column-walk backward (scan_bwd_cw.cuh) on the forward's block states: eligibility, argument block, tensor maps (u, delta,
+// dout, du, ddelta; not encoded when tm is null).
 bool plan_cw_bwd(const mia_ss_params &p, const DeviceInfo &di, mia::CwBwdArgs &r, CUtensorMap *tm, int &grid) {
     const int es = esize(p.itype), eo = esize(p.otype), L = p.seqlen;
     int g = 0;
-    if (!p.hblk || !cw_geometry(p, di.sms, g)) return false;
-    if (dbg_knob("MIA_NO_CW_BWD")) return false;
-    const int rpg = p.dim / p.n_groups;
-    auto dense = [&](long long bs, long long ds) { return ds == L && bs == (long long)p.dim * L; };
-    if (!dense(p.u_batch_stride, p.u_d_stride) || !dense(p.delta_batch_stride, p.delta_d_stride) ||
-        !dense(p.dout_batch_stride, p.dout_d_stride) || !dense(p.du_batch_stride, p.du_d_stride) ||
-        !dense(p.ddelta_batch_stride, p.ddelta_d_stride)) return false;
-    if (p.A_d_stride != 1 && p.dim > 1) return false;
-    if (((uintptr_t)p.u | (uintptr_t)p.delta | (uintptr_t)p.dout | (uintptr_t)p.du | (uintptr_t)p.ddelta) & 15) return false;
+    if (!p.hblk || !cw_geometry(p, di.sms, g) || dbg_knob("MIA_NO_CW_BWD")) return false;
+    // Short rows always; rows of more than one 256-token chunk only with enough 32-row items to fill the SMs.  Measured
+    // (B200, runs r2i / r2n, L = 6400, bf16): B = 16 (1536 items) 0.86 ms against 1.77 ms for the warp-scan kernel; B = 4 (384
+    // items = 2.6 warps per SM): a one-warp-per-item walk took 0.75 ms against 0.55 ms.
+    const long long items32 = (long long)p.batch * (p.dim / 32);
+    if (!(L <= mia::kRowsChunk || items32 >= 4LL * di.sms || dbg_knob("MIA_FORCE_CW_BWD"))) return false;
+    if (!bwd_rows_dense(p) || !a_per_row(p) || !aligned16({p.u, p.delta, p.dout, p.du, p.ddelta})) return false;
     const unsigned long long trows = (unsigned long long)p.batch * p.dim / g, tcols = (unsigned long long)g * L;
     if (tcols >= (1ull << 31) || trows >= (1ull << 31)) return false;
-    memset(&r, 0, sizeof(r));
-    r.batch = p.batch; r.dim = p.dim; r.L = L; r.G = p.n_groups; r.rows_per_group = rpg; r.softplus = p.delta_softplus;
+    if ((((uintptr_t)p.B | (uintptr_t)p.C) & 3) || ((p.B_batch_stride | p.B_group_stride | p.C_batch_stride | p.C_group_stride) * es) % 4) return false;
+    init_args(r, p);
     r.g = g;
-    r.n_items = p.batch * p.n_groups * (rpg / (32 * g));
+    r.n_items = p.batch * p.n_groups * (r.rows_per_group / (32 * g));
     r.ngrp = (g * L + mia::kCwGrp - 1) / mia::kCwGrp;
     r.nwin = (g * L + mia::kCwWin - 1) / mia::kCwWin;
     const int tile_i = 32 * mia::kCwWin * es, tile_o = 32 * mia::kCwWin * eo;
@@ -606,17 +581,14 @@ bool plan_cw_bwd(const mia_ss_params &p, const DeviceInfo &di, mia::CwBwdArgs &r
     r.off_red = r.off_pf + 1024;                                // [32][20] fp32 scratch of the row reductions
     r.off_bar = r.off_red + 32 * 20 * 4;
     r.smem_bytes = r.off_bar + 8 * r.ns + 16;
-    if ((((uintptr_t)p.B | (uintptr_t)p.C) & 3) || ((p.B_batch_stride | p.B_group_stride | p.C_batch_stride | p.C_group_stride) * es) % 4) return false;
-    r.A = p.A; r.B = p.B; r.C = p.C; r.D = p.D; r.delta_bias = p.delta_bias; r.hblk = p.hblk;
-    r.B_bs = p.B_batch_stride; r.B_gs = p.B_group_stride; r.C_bs = p.C_batch_stride; r.C_gs = p.C_group_stride;
+    r.hblk = p.hblk;
     const void *ptrs[5] = {p.u, p.delta, p.dout, p.du, p.ddelta};
-    for (int i = 0; i < 5; ++i) {
+    for (int i = 0; tm && i < 5; ++i) {
         const int e = i == 2 ? eo : es;
         const int trc = mia::tma_make_2d(&tm[i], ptrs[i], trows, tcols, tcols * e, 32, mia::kCwWin, e, mia::kCwWin * e);
         if (trc != 0) { MIA_TRACE("cw bwd: tensor map %d rejected (CUresult %d)", i, trc); return false; }
     }
-    int per_sm = (227 * 1024) / (r.smem_bytes + 1024);
-    if (per_sm > 12) per_sm = 12;                               // 32 threads x 168 registers: 3 warps per scheduler
+    int per_sm = resident_ctas(r.smem_bytes, 12);               // 32 threads x 168 registers: 3 warps per scheduler
     // Many short items: 8 resident warps per SM finish an item 1.8x faster than 12 do (measured, gpurun r2s / r2t, bf16,
     // B = 148: L = 196 0.313 against 0.354 ms, L = 200 0.302 / 0.362, L = 100 0.173 / 0.193, L = 104 0.173 / 0.184), so with
     // at least two rounds of short rows the extra rounds cost less than the contention.  Long rows (L = 1024, B = 32: 0.341
@@ -633,26 +605,17 @@ bool plan_cw_bwd(const mia_ss_params &p, const DeviceInfo &di, mia::CwBwdArgs &r
     return true;
 }
 
-// Deterministic d_state 16 backward (scan_bwd_rowsn.cuh): eligibility + argument block.
+// Deterministic d_state 16 backward (scan_bwd_rowsn.cuh).
 bool plan_rowsn_bwd(const mia_ss_params &p, const DeviceInfo &di, mia::RowsNBwdArgs &r, int &grid) {
     const int es = esize(p.itype), eo = esize(p.otype), L = p.seqlen;
-    const int rpg = p.dim / p.n_groups;
     RowsNSplit sp;
-    if (!rowsn_bwd_split(p, di.sms, kRowsNCtasPerSm, sp)) return false;
-    if (dbg_knob("MIA_NO_ROWS_BWD")) return false;
-    auto dense = [&](long long bs, long long ds) { return ds == L && bs == (long long)p.dim * L; };
-    if (!dense(p.u_batch_stride, p.u_d_stride) || !dense(p.delta_batch_stride, p.delta_d_stride) ||
-        !dense(p.dout_batch_stride, p.dout_d_stride) || !dense(p.du_batch_stride, p.du_d_stride) ||
-        !dense(p.ddelta_batch_stride, p.ddelta_d_stride)) return false;
-    if (((uintptr_t)p.u | (uintptr_t)p.delta | (uintptr_t)p.dout) & 15) return false;
-    if (p.z) {
-        if (!dense(p.z_batch_stride, p.z_d_stride) || !dense(p.out_saved_batch_stride, p.out_saved_d_stride) ||
-            !dense(p.dz_batch_stride, p.dz_d_stride)) return false;
-        if (((uintptr_t)p.z | (uintptr_t)p.out_saved) & 15) return false;
-    }
-    memset(&r, 0, sizeof(r));
-    r.batch = p.batch; r.dim = p.dim; r.L = L; r.G = p.n_groups; r.rows_per_group = rpg;
-    r.softplus = p.delta_softplus; r.has_z = p.z != nullptr;
+    if (!rowsn_bwd_split(p, di.sms, kRowsNCtasPerSm, sp) || dbg_knob("MIA_NO_ROWS_BWD")) return false;
+    if (!bwd_rows_dense(p) || !aligned16({p.u, p.delta, p.dout})) return false;
+    if (p.z && (!dense_rows(p, {{p.z_batch_stride, p.z_d_stride}, {p.out_saved_batch_stride, p.out_saved_d_stride}, {p.dz_batch_stride, p.dz_d_stride}}) ||
+                !aligned16({p.z, p.out_saved})))
+        return false;
+    init_args(r, p);
+    r.has_z = p.z != nullptr;
     r.n_oct = sp.n_oct; r.oct_per_cta = sp.oct_per_cta; r.oct_per_group = sp.oct_per_group; r.max_parts = sp.max_parts;
     r.nblk = (L + mia::kRnBlk - 1) / mia::kRnBlk;
     r.Lp = r.nblk * mia::kRnBlk;
@@ -680,17 +643,141 @@ bool plan_rowsn_bwd(const mia_ss_params &p, const DeviceInfo &di, mia::RowsNBwdA
     r.off_bar = take(8);
     r.smem_bytes = off;
     if (r.smem_bytes > di.smem_optin) return false;
-    r.u = p.u; r.delta = p.delta; r.A = p.A; r.B = p.B; r.C = p.C; r.D = p.D; r.delta_bias = p.delta_bias; r.dout = p.dout;
-    r.z = p.z; r.out_saved = p.out_saved; r.du = p.du; r.ddelta = p.ddelta; r.dz = p.dz;
-    r.A_ds = p.A_d_stride; r.A_ns = p.A_dstate_stride;
-    r.B_bs = p.B_batch_stride; r.B_gs = p.B_group_stride; r.B_ns = p.B_dstate_stride;
-    r.C_bs = p.C_batch_stride; r.C_gs = p.C_group_stride; r.C_ns = p.C_dstate_stride;
+    r.u = p.u; r.delta = p.delta; r.dout = p.dout; r.z = p.z; r.out_saved = p.out_saved; r.du = p.du; r.ddelta = p.ddelta; r.dz = p.dz;
+    r.A_ds = p.A_d_stride; r.A_ns = p.A_dstate_stride; r.B_ns = p.B_dstate_stride; r.C_ns = p.C_dstate_stride;
     grid = sp.grid;
     return true;
 }
 
+// ---- Selection: one plan per call and direction, shared by the calls, mia_ss_describe_plan and mia_ss_fwd_writes_block_states.
+enum Family { kCw, kChunks, kRows, kStream, kRowsN, kWarpScan };
+const char *const kFamilyName[] = {"cw", "chunks", "rows", "stream", "rowsn", "warp_scan"};
+
+struct FwdPlan {
+    Family family;
+    int grid, smem;
+    mia::CwFwdArgs cw;
+    mia::ChunkArgs chunks;
+    mia::RowsArgs rows;
+    mia::StreamArgs stream;
+    mia::RowsNArgs rowsn;
+    mia::ScanArgs ws;
+    CUtensorMap tm[3];
+    int launches() const { return family == kChunks ? 3 : 1; }   // the chunk-parallel forward is three kernels
+};
+
+// The first family, in order of preference, that takes the shape; the warp-scan kernels take every valid one.
+// encode = false: the column-walk tensor maps are not encoded (assumed encodable).  When encoding fails the next family runs.
+int plan_fwd(const mia_ss_params &p, const DeviceInfo &di, bool encode, FwdPlan &f) {
+    if (plan_cw_fwd(p, di, f.cw, encode ? f.tm : nullptr, f.grid)) { f.family = kCw; f.smem = f.cw.smem_bytes; return MIA_OK; }
+    if (plan_chunks_fwd(p, di, f.chunks, f.grid)) { f.family = kChunks; f.smem = f.chunks.smem_bytes; return MIA_OK; }
+    if (plan_rows_fwd(p, di, f.rows, f.grid)) { f.family = kRows; f.smem = f.rows.smem_bytes; return MIA_OK; }
+    if (plan_stream_fwd(p, di, f.stream, f.grid)) { f.family = kStream; f.smem = f.stream.smem_bytes; return MIA_OK; }
+    if (plan_rowsn_fwd(p, di, f.rowsn, f.grid)) { f.family = kRowsN; f.smem = f.rowsn.smem_bytes; return MIA_OK; }
+    Plan pl;
+    mia::ScanArgs &a = f.ws;
+    if (int rc = plan_and_layout(p, di, false, pl, a)) return rc;
+    a.out = p.out; a.out_z = p.out_z;
+    a.out_bs = p.out_batch_stride; a.out_ds = p.out_d_stride; a.outz_bs = p.out_z_batch_stride; a.outz_ds = p.out_z_d_stride;
+    f.family = kWarpScan;
+    f.grid = a.n_seg < di.sms ? a.n_seg : di.sms;
+    f.smem = a.smem_bytes;
+    return MIA_OK;
+}
+
+struct BwdPlan {
+    Family family;
+    int grid, smem;
+    mia::CwBwdArgs cw;
+    mia::RowsNBwdArgs rowsn;
+    mia::RowsBwdArgs rows;
+    mia::ScanArgs ws;                 // planned for every call: its work split sizes the workspace
+    CUtensorMap tm[5];
+    WorkspaceLayout w;
+    int parts;                        // dB / dC partial slots per (batch, group) that the finalize folds
+    bool atomic;                      // dB / dC accumulate with red.add into the zeroed acc_dB / acc_dC (two memsets)
+    int launches() const { return 2 + (atomic ? 2 : 0); }
+};
+
+template <typename R>
+void set_partials(R &r, const mia::ScanArgs &a) {
+    r.part_dA = a.part_dA; r.part_dD = a.part_dD; r.part_dbias = a.part_dbias; r.acc_dB = a.acc_dB; r.acc_dC = a.acc_dC;
+}
+
+// The deterministic d_state 16 kernel first, then the column-walk kernel on the forward's block states, the row-serial
+// kernel, and the warp-scan kernels for every other valid shape.  Checks the workspace like the call.
+int plan_bwd(const mia_ss_params &p, const DeviceInfo &di, bool encode, BwdPlan &b) {
+    Plan pl;
+    mia::ScanArgs &a = b.ws;
+    if (int rc = plan_and_layout(p, di, true, pl, a)) return rc;
+    a.dout = p.dout; a.out_saved = p.out_saved; a.du = p.du; a.ddelta = p.ddelta; a.dz = p.dz;
+    a.dout_bs = p.dout_batch_stride; a.dout_ds = p.dout_d_stride;
+    a.osaved_bs = p.out_saved_batch_stride; a.osaved_ds = p.out_saved_d_stride;
+    a.du_bs = p.du_batch_stride; a.du_ds = p.du_d_stride; a.dd_bs = p.ddelta_batch_stride; a.dd_ds = p.ddelta_d_stride;
+    a.dz_bs = p.dz_batch_stride; a.dz_ds = p.dz_d_stride;
+    const WorkspaceLayout &w = b.w = workspace_layout(p, pl, di.sms);
+    if (!p.workspace || p.workspace_bytes < w.total)
+        return fail(MIA_EWORKSPACE, "workspace too small: need %zu bytes, got %zu", w.total, p.workspace ? p.workspace_bytes : (size_t)0);
+    MIA_CHECK(((uintptr_t)p.workspace & 255) == 0, "workspace must be 256-byte aligned");
+    char *ws = (char *)p.workspace;
+    a.part_dA = (float *)(ws + w.part_dA); a.part_dD = (float *)(ws + w.part_dD); a.part_dbias = (float *)(ws + w.part_dbias);
+    a.acc_dB = (float *)(ws + w.acc_dB); a.acc_dC = (float *)(ws + w.acc_dC);
+    a.ddelta_full = (float *)(ws + w.ddelta_full);
+    if (plan_rowsn_bwd(p, di, b.rowsn, b.grid)) {
+        b.family = kRowsN; b.smem = b.rowsn.smem_bytes; b.parts = b.rowsn.max_parts;
+    } else if (plan_cw_bwd(p, di, b.cw, encode ? b.tm : nullptr, b.grid)) {
+        b.family = kCw; b.smem = b.cw.smem_bytes; b.parts = b.cw.rows_per_group / 32;
+    } else if (plan_rows_bwd(p, di, b.rows, b.grid)) {
+        b.family = kRows; b.smem = b.rows.smem_bytes; b.parts = b.rows.rows_per_group / 32;
+    } else {
+        b.family = kWarpScan; b.grid = a.n_seg < di.sms ? a.n_seg : di.sms; b.smem = a.smem_bytes; b.parts = pl.split;
+    }
+    set_partials(b.cw, a);
+    set_partials(b.rowsn, a);
+    set_partials(b.rows, a);
+    b.atomic = w.bc_atomic && b.family != kRowsN;
+    a.bc_atomic = b.atomic;
+    return MIA_OK;
+}
+
+// The key=value line of mia_ss_describe_plan.
+void describe(const FwdPlan &f, char *buf, size_t n) {
+    char geo[96] = "";
+    if (f.family == kCw) snprintf(geo, sizeof(geo), " g=%d ns=%d", f.cw.g, f.cw.ns);
+    if (f.family == kWarpScan) snprintf(geo, sizeof(geo), " LPR=%d split=%d RT=%d stages=%d", f.ws.LPR, f.ws.split, f.ws.RT, f.ws.stages);
+    snprintf(buf, n, "kernel=%s grid=%d smem=%d%s launches=%d", kFamilyName[f.family], f.grid, f.smem, geo, f.launches());
+}
+void describe(const BwdPlan &b, char *buf, size_t n) {
+    char geo[96] = "";
+    if (b.family == kCw) snprintf(geo, sizeof(geo), " g=%d ns=%d wide=%d", b.cw.g, b.cw.ns, b.cw.wide);
+    if (b.family == kWarpScan) snprintf(geo, sizeof(geo), " LPR=%d split=%d RT=%d stages=%d", b.ws.LPR, b.ws.split, b.ws.RT, b.ws.stages);
+    snprintf(buf, n, "kernel=%s grid=%d smem=%d%s parts=%d atomic=%d launches=%d", kFamilyName[b.family], b.grid, b.smem, geo, b.parts,
+             b.atomic ? 1 : 0, b.launches());
+}
+
+int validate_fwd(const mia_ss_params *pp) {
+    if (!pp) return fail(MIA_EINVAL, "null params");
+    const mia_ss_params &p = *pp;
+    if (int rc = validate_common(p)) return rc;
+    MIA_CHECK(p.out && p.x, "out and x must not be null");
+    MIA_CHECK(!p.z || p.out_z, "out_z is required when z is given");
+    return MIA_OK;
+}
+
+int validate_bwd(const mia_ss_params *pp) {
+    if (!pp) return fail(MIA_EINVAL, "null params");
+    const mia_ss_params &p = *pp;
+    if (int rc = validate_common(p)) return rc;
+    MIA_CHECK(p.dout && p.du && p.ddelta && p.dA && p.dB && p.dC, "dout, du, ddelta, dA, dB, dC must not be null");
+    MIA_CHECK(!p.D || p.dD, "dD is required when D is given");
+    MIA_CHECK(!p.delta_bias || p.ddelta_bias, "ddelta_bias is required when delta_bias is given");
+    MIA_CHECK(!p.z || (p.dz && p.out_saved), "dz and out_saved are required when z is given");
+    MIA_CHECK(p.n_chunks == 1 || p.x, "x is required when the sequence spans more than one chunk");
+    return MIA_OK;
+}
+
 template <typename F>
-int dispatch(int itype, F &&f) {
+auto dispatch(int itype, F &&f) {
     switch (itype) {
         case MIA_F32: return f((float *)nullptr);
         case MIA_F16: return f((__half *)nullptr);
@@ -814,105 +901,58 @@ int mia_ss_fwd_writes_block_states(const mia_ss_params *pp) {
     if (!pp || !pp->hblk || validate_sizes(*pp) != MIA_OK || !pp->u || !pp->delta || !pp->out) return 0;
     DeviceInfo di;
     if (device_info(di) != MIA_OK) return 0;
-    mia::CwFwdArgs rw;
-    CUtensorMap tm[3];
-    int grid = 0;
-    return plan_cw_fwd(*pp, di, rw, tm, grid) ? 1 : 0;          // the column-walk forward is the kernel that fills hblk
+    FwdPlan f;                                                   // the maps are encoded: a map the driver rejects means no cw
+    return plan_fwd(*pp, di, true, f) == MIA_OK && f.family == kCw ? 1 : 0;   // the column-walk forward is the kernel that fills hblk
+}
+
+int mia_ss_describe_plan(const mia_ss_params *pp, int backward, int sms, int smem_optin, char *buf, size_t buf_len) {
+    if (int rc = backward ? validate_bwd(pp) : validate_fwd(pp)) return rc;
+    MIA_CHECK(buf && buf_len > 0, "no buffer for the plan");
+    DeviceInfo di;
+    if (sms <= 0 || smem_optin <= 0) {
+        if (int rc = device_info(di)) return rc;
+    }
+    if (sms > 0) di.sms = sms;
+    if (smem_optin > 0) di.smem_optin = smem_optin;
+    if (backward) {
+        BwdPlan b;
+        if (int rc = plan_bwd(*pp, di, false, b)) return rc;
+        describe(b, buf, buf_len);
+    } else {
+        FwdPlan f;
+        if (int rc = plan_fwd(*pp, di, false, f)) return rc;
+        describe(f, buf, buf_len);
+    }
+    return MIA_OK;
 }
 
 int mia_selective_scan_fwd(const mia_ss_params *pp, void *cuda_stream) {
-    if (!pp) return fail(MIA_EINVAL, "null params");
+    if (int rc = validate_fwd(pp)) return rc;
     const mia_ss_params &p = *pp;
-    if (int rc = validate_common(p)) return rc;
-    MIA_CHECK(p.out && p.x, "out and x must not be null");
-    MIA_CHECK(!p.z || p.out_z, "out_z is required when z is given");
     DeviceInfo di;
     if (int rc = device_info(di)) return rc;
+    FwdPlan f;
+    if (int rc = plan_fwd(p, di, true, f)) return rc;
+#ifdef MIA_DEBUG
+    char line[256];
+    describe(f, line, sizeof(line));
+    MIA_TRACE("fwd: %s", line);
+#endif
     cudaStream_t stream = (cudaStream_t)cuda_stream;
-    {
-        mia::CwFwdArgs r;
-        CUtensorMap tm[3];
-        int rgrid = 0;
-        if (plan_cw_fwd(p, di, r, tm, rgrid)) {
-            MIA_TRACE("fwd: cw g=%d ns=%d nwin=%d grid=%d smem=%d", r.g, r.ns, r.nwin, rgrid, r.smem_bytes);
-            const bool of32 = p.otype == MIA_F32 && p.itype != MIA_F32;
-            const int rc = dispatch(p.itype, [&](auto *tag) {
-                using T = typename std::remove_pointer<decltype(tag)>::type;
-                return (int)mia::launch_fwd_cw<T>(tm, r, rgrid, of32, stream);
-            });
-            if (rc != 0) return fail(MIA_ECUDA, "selective_scan_fwd (column-walk) launch: %s", cudaGetErrorString((cudaError_t)rc));
-            g_launches.fetch_add(1);
-            return MIA_OK;
-        }
-    }
-    {
-        mia::ChunkArgs r;
-        int rgrid = 0;
-        if (plan_chunks_fwd(p, di, r, rgrid)) {
-            const bool of32 = p.otype == MIA_F32 && p.itype != MIA_F32;
-            const int rc = dispatch(p.itype, [&](auto *tag) {
-                using T = typename std::remove_pointer<decltype(tag)>::type;
-                return (int)mia::launch_fwd_chunks<T>(r, rgrid, of32, stream);
-            });
-            if (rc != 0) return fail(MIA_ECUDA, "selective_scan_fwd (chunk-parallel) launch: %s", cudaGetErrorString((cudaError_t)rc));
-            g_launches.fetch_add(3);
-            return MIA_OK;
-        }
-    }
-    {
-        mia::RowsArgs r;
-        int rgrid = 0;
-        if (plan_rows_fwd(p, di, r, rgrid)) {
-            const bool of32 = p.otype == MIA_F32 && p.itype != MIA_F32;
-            const int rc = dispatch(p.itype, [&](auto *tag) {
-                using T = typename std::remove_pointer<decltype(tag)>::type;
-                return (int)mia::launch_fwd_rows<T>(r, rgrid, of32, stream);
-            });
-            if (rc != 0) return fail(MIA_ECUDA, "selective_scan_fwd (row-serial) launch: %s", cudaGetErrorString((cudaError_t)rc));
-            g_launches.fetch_add(1);
-            return MIA_OK;
-        }
-    }
-    {
-        mia::StreamArgs r;
-        int rgrid = 0;
-        if (plan_stream_fwd(p, di, r, rgrid)) {
-            const bool of32 = p.otype == MIA_F32 && p.itype != MIA_F32;
-            const int rc = dispatch(p.itype, [&](auto *tag) {
-                using T = typename std::remove_pointer<decltype(tag)>::type;
-                return (int)mia::launch_fwd_stream<T>(r, rgrid, of32, stream);
-            });
-            if (rc != 0) return fail(MIA_ECUDA, "selective_scan_fwd (streaming) launch: %s", cudaGetErrorString((cudaError_t)rc));
-            g_launches.fetch_add(1);
-            return MIA_OK;
-        }
-    }
-    {
-        mia::RowsNArgs r;
-        int rgrid = 0;
-        if (plan_rowsn_fwd(p, di, r, rgrid)) {
-            const bool of32 = p.otype == MIA_F32 && p.itype != MIA_F32;
-            const int rc = dispatch(p.itype, [&](auto *tag) {
-                using T = typename std::remove_pointer<decltype(tag)>::type;
-                return (int)mia::launch_fwd_rowsn<T>(r, rgrid, of32, stream);
-            });
-            if (rc != 0) return fail(MIA_ECUDA, "selective_scan_fwd (row-serial, d_state %d) launch: %s", p.dstate, cudaGetErrorString((cudaError_t)rc));
-            g_launches.fetch_add(1);
-            return MIA_OK;
-        }
-    }
-    Plan pl;
-    mia::ScanArgs a;
-    if (int rc = plan_and_layout(p, di, false, pl, a)) return rc;
-    a.out = p.out; a.out_z = p.out_z;
-    a.out_bs = p.out_batch_stride; a.out_ds = p.out_d_stride; a.outz_bs = p.out_z_batch_stride; a.outz_ds = p.out_z_d_stride;
-    const int grid = a.n_seg < di.sms ? a.n_seg : di.sms;
-    const int rc = dispatch(p.itype, [&](auto *tag) {
+    const bool of32 = p.otype == MIA_F32 && p.itype != MIA_F32;
+    const cudaError_t rc = dispatch(p.itype, [&](auto *tag) {
         using T = typename std::remove_pointer<decltype(tag)>::type;
-        return (int)mia::launch_fwd_any<T>(a, grid, stream);
+        switch (f.family) {
+            case kCw: return mia::launch_fwd_cw<T>(f.tm, f.cw, f.grid, of32, stream);
+            case kChunks: return mia::launch_fwd_chunks<T>(f.chunks, f.grid, of32, stream);
+            case kRows: return mia::launch_fwd_rows<T>(f.rows, f.grid, of32, stream);
+            case kStream: return mia::launch_fwd_stream<T>(f.stream, f.grid, of32, stream);
+            case kRowsN: return mia::launch_fwd_rowsn<T>(f.rowsn, f.grid, of32, stream);
+            default: return mia::launch_fwd_any<T>(f.ws, f.grid, stream);
+        }
     });
-    if (rc != 0) return fail(MIA_ECUDA, "selective_scan_fwd launch: %s", cudaGetErrorString((cudaError_t)rc));
-    g_launches.fetch_add(1);
+    if (rc != cudaSuccess) return fail(MIA_ECUDA, "selective_scan_fwd (%s kernel) launch: %s", kFamilyName[f.family], cudaGetErrorString(rc));
+    g_launches.fetch_add(f.launches());
     return MIA_OK;
 }
 
@@ -928,94 +968,42 @@ size_t mia_selective_scan_bwd_workspace(const mia_ss_params *pp) {
 }
 
 int mia_selective_scan_bwd(const mia_ss_params *pp, void *cuda_stream) {
-    if (!pp) return fail(MIA_EINVAL, "null params");
+    if (int rc = validate_bwd(pp)) return rc;
     const mia_ss_params &p = *pp;
-    if (int rc = validate_common(p)) return rc;
-    MIA_CHECK(p.dout && p.du && p.ddelta && p.dA && p.dB && p.dC, "dout, du, ddelta, dA, dB, dC must not be null");
-    MIA_CHECK(!p.D || p.dD, "dD is required when D is given");
-    MIA_CHECK(!p.delta_bias || p.ddelta_bias, "ddelta_bias is required when delta_bias is given");
-    MIA_CHECK(!p.z || (p.dz && p.out_saved), "dz and out_saved are required when z is given");
-    MIA_CHECK(p.n_chunks == 1 || p.x, "x is required when the sequence spans more than one chunk");
     DeviceInfo di;
     if (int rc = device_info(di)) return rc;
-    Plan pl;
-    mia::ScanArgs a;
-    if (int rc = plan_and_layout(p, di, true, pl, a)) return rc;
-    a.dout = p.dout; a.out_saved = p.out_saved; a.du = p.du; a.ddelta = p.ddelta; a.dz = p.dz;
-    a.dout_bs = p.dout_batch_stride; a.dout_ds = p.dout_d_stride;
-    a.osaved_bs = p.out_saved_batch_stride; a.osaved_ds = p.out_saved_d_stride;
-    a.du_bs = p.du_batch_stride; a.du_ds = p.du_d_stride; a.dd_bs = p.ddelta_batch_stride; a.dd_ds = p.ddelta_d_stride;
-    a.dz_bs = p.dz_batch_stride; a.dz_ds = p.dz_d_stride;
-    const WorkspaceLayout w = workspace_layout(p, pl, di.sms);
-    if (!p.workspace || p.workspace_bytes < w.total)
-        return fail(MIA_EWORKSPACE, "workspace too small: need %zu bytes, got %zu", w.total, p.workspace ? p.workspace_bytes : (size_t)0);
-    MIA_CHECK(((uintptr_t)p.workspace & 255) == 0, "workspace must be 256-byte aligned");
-    char *ws = (char *)p.workspace;
-    a.part_dA = (float *)(ws + w.part_dA); a.part_dD = (float *)(ws + w.part_dD); a.part_dbias = (float *)(ws + w.part_dbias);
-    a.acc_dB = (float *)(ws + w.acc_dB); a.acc_dC = (float *)(ws + w.acc_dC);
-    a.ddelta_full = (float *)(ws + w.ddelta_full);
-    a.bc_atomic = w.bc_atomic;
+    BwdPlan b;
+    if (int rc = plan_bwd(p, di, true, b)) return rc;
+#ifdef MIA_DEBUG
+    char line[256];
+    describe(b, line, sizeof(line));
+    MIA_TRACE("bwd: %s", line);
+#endif
+    const mia::ScanArgs &a = b.ws;
     cudaStream_t stream = (cudaStream_t)cuda_stream;
-    mia::RowsNBwdArgs rn;
-    int rn_grid = 0;
-    const bool use_rowsn = plan_rowsn_bwd(p, di, rn, rn_grid);
-    if (use_rowsn) a.bc_atomic = 0;
-    if (a.bc_atomic) {
-        MIA_CUDA(cudaMemsetAsync(a.acc_dB, 0, w.acc_bytes, stream));
-        MIA_CUDA(cudaMemsetAsync(a.acc_dC, 0, w.acc_bytes, stream));
+    if (b.atomic) {
+        MIA_CUDA(cudaMemsetAsync(a.acc_dB, 0, b.w.acc_bytes, stream));
+        MIA_CUDA(cudaMemsetAsync(a.acc_dC, 0, b.w.acc_bytes, stream));
         g_launches.fetch_add(2);
     }
-    int rc = 0, bc_parts = pl.split;
-    mia::RowsBwdArgs rb;
-    int rgrid = 0;
-    CUtensorMap tmaps[5];
-    // Column-walk kernel (one warp per 32 g rows, phase 2 only, on the forward's block states): short rows always; rows of more
-    // than one 256-token chunk only with enough 32-row items to fill the SMs.  Measured (gpurun r2i / r2n, L = 6400, bf16):
-    // B = 16 (1536 items) 0.86 ms against 1.77 ms for the warp-scan kernel; B = 4 (384 items = 2.6 warps per SM): a one-warp-
-    // per-item walk took 0.75 ms against 0.55 ms.
-    const long long items32 = (long long)p.batch * (p.dim / 32);
-    mia::CwBwdArgs cwb;
-    const bool want_cw = !use_rowsn && p.hblk && (p.seqlen <= mia::kRowsChunk || items32 >= 4LL * di.sms || dbg_knob("MIA_FORCE_CW_BWD"));
-    if (want_cw && plan_cw_bwd(p, di, cwb, tmaps, rgrid)) {
-        MIA_TRACE("bwd: cw g=%d ns=%d ngrp=%d grid=%d smem=%d", cwb.g, cwb.ns, cwb.ngrp, rgrid, cwb.smem_bytes);
-        cwb.part_dA = a.part_dA; cwb.part_dD = a.part_dD; cwb.part_dbias = a.part_dbias; cwb.acc_dB = a.acc_dB; cwb.acc_dC = a.acc_dC;
-        bc_parts = cwb.rows_per_group / 32;
-        const bool of32 = p.otype == MIA_F32 && p.itype != MIA_F32;
-        rc = dispatch(p.itype, [&](auto *tag) {
-            using T = typename std::remove_pointer<decltype(tag)>::type;
-            return (int)mia::launch_bwd_cw<T>(tmaps, cwb, rgrid, of32, stream);
-        });
-    } else if (use_rowsn) {
-        rn.part_dA = a.part_dA; rn.part_dD = a.part_dD; rn.part_dbias = a.part_dbias; rn.acc_dB = a.acc_dB; rn.acc_dC = a.acc_dC;
-        bc_parts = rn.max_parts;
-        const bool of32 = p.otype == MIA_F32 && p.itype != MIA_F32;
-        rc = dispatch(p.itype, [&](auto *tag) {
-            using T = typename std::remove_pointer<decltype(tag)>::type;
-            return (int)mia::launch_bwd_rowsn<T>(rn, rn_grid, of32, stream);
-        });
-    } else if (plan_rows_bwd(p, di, rb, rgrid)) {
-        rb.part_dA = a.part_dA; rb.part_dD = a.part_dD; rb.part_dbias = a.part_dbias; rb.acc_dB = a.acc_dB; rb.acc_dC = a.acc_dC;
-        bc_parts = rb.rows_per_group / 32;
-        const bool of32 = p.otype == MIA_F32 && p.itype != MIA_F32;
-        rc = dispatch(p.itype, [&](auto *tag) {
-            using T = typename std::remove_pointer<decltype(tag)>::type;
-            return (int)mia::launch_bwd_rows<T>(rb, rgrid, of32, stream);
-        });
-    } else {
-        const int grid = a.n_seg < di.sms ? a.n_seg : di.sms;
-        rc = dispatch(p.itype, [&](auto *tag) {
-            using T = typename std::remove_pointer<decltype(tag)>::type;
-            return (int)mia::launch_bwd_any<T>(a, grid, stream);
-        });
-    }
-    if (rc != 0) return fail(MIA_ECUDA, "selective_scan_bwd launch: %s", cudaGetErrorString((cudaError_t)rc));
+    const bool of32 = p.otype == MIA_F32 && p.itype != MIA_F32;
+    cudaError_t rc = dispatch(p.itype, [&](auto *tag) {
+        using T = typename std::remove_pointer<decltype(tag)>::type;
+        switch (b.family) {
+            case kCw: return mia::launch_bwd_cw<T>(b.tm, b.cw, b.grid, of32, stream);
+            case kRowsN: return mia::launch_bwd_rowsn<T>(b.rowsn, b.grid, of32, stream);
+            case kRows: return mia::launch_bwd_rows<T>(b.rows, b.grid, of32, stream);
+            default: return mia::launch_bwd_any<T>(a, b.grid, stream);
+        }
+    });
+    if (rc != cudaSuccess) return fail(MIA_ECUDA, "selective_scan_bwd (%s kernel) launch: %s", kFamilyName[b.family], cudaGetErrorString(rc));
     g_launches.fetch_add(1);
 
     FinArgs f;
     memset(&f, 0, sizeof(f));
     f.batch = p.batch; f.dim = p.dim; f.L = p.seqlen; f.N = p.dstate; f.G = p.n_groups; f.delta_dim = p.delta_dim;
-    f.ratio = p.dim / p.delta_dim; f.tiles = bc_parts; f.bc_atomic = a.bc_atomic; f.Lp = (p.seqlen + 3) & ~3;
-    if (use_rowsn) { f.oct_per_cta = rn.oct_per_cta; f.oct_per_group = rn.oct_per_group; }
+    f.ratio = p.dim / p.delta_dim; f.tiles = b.parts; f.bc_atomic = b.atomic; f.Lp = (p.seqlen + 3) & ~3;
+    if (b.family == kRowsN) { f.oct_per_cta = b.rowsn.oct_per_cta; f.oct_per_group = b.rowsn.oct_per_group; }
     f.part_dA = a.part_dA; f.part_dD = a.part_dD; f.part_dbias = a.part_dbias; f.acc_dB = a.acc_dB; f.acc_dC = a.acc_dC;
     f.ddelta_full = a.ddelta_full;
     f.dA = p.dA; f.dD = p.dD; f.dbias = p.ddelta_bias; f.dB = p.dB; f.dC = p.dC; f.ddelta = p.ddelta;
@@ -1034,9 +1022,9 @@ int mia_selective_scan_bwd(const mia_ss_params *pp, void *cuda_stream) {
     rc = dispatch(p.itype, [&](auto *tag) {
         using T = typename std::remove_pointer<decltype(tag)>::type;
         ss_finalize_kernel<T><<<(int)blocks, 256, 0, stream>>>(f);
-        return (int)cudaGetLastError();
+        return cudaGetLastError();
     });
-    if (rc != 0) return fail(MIA_ECUDA, "selective_scan_bwd finalize launch: %s", cudaGetErrorString((cudaError_t)rc));
+    if (rc != cudaSuccess) return fail(MIA_ECUDA, "selective_scan_bwd finalize launch: %s", cudaGetErrorString(rc));
     g_launches.fetch_add(1);
     return MIA_OK;
 }

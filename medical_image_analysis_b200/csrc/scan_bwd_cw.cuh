@@ -31,20 +31,6 @@ namespace mia {
 #ifndef MIA_CW_FMA
 #define MIA_CW_FMA 0             // 1: h_t by one FFMA (a_t h_{t-1} off the serial chain); measured slower in the 168-register build (tools/ab_cw.py)
 #endif
-constexpr int kCwGrp = 16;       // columns per group = tokens per recompute block
-constexpr int kCwWin = 32;       // columns per window = per stage of the ring (two groups)
-
-struct CwBwdArgs {
-    int batch, dim, L, G, rows_per_group;
-    int softplus;
-    int g, n_items, ngrp, nwin, ns;         // rows per tensor-map row; items of 32 g rows; 16-column groups / 32-column windows per tensor-map row; stages
-    int wide;                               // at most 8 resident warps per SM planned: the build with up to 255 registers per thread
-    int stage_bytes, off_bc32, off_pf, off_red, off_bar, smem_bytes;
-    const void *A, *B, *C, *D, *delta_bias;
-    const float *hblk;
-    float *part_dA, *part_dD, *part_dbias, *acc_dB, *acc_dC;
-    long long B_bs, B_gs, C_bs, C_gs;
-};
 
 struct CwRegs {
     float2 a[8], hp[8], m[8];      // a_t, a_t h_{t-1}, softplus(delta + bias) log2e of the 16 tokens

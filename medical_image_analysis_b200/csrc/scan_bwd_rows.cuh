@@ -28,24 +28,6 @@
 
 namespace mia {
 
-constexpr int kBlk = 16;   // tokens per recompute block (= values per quantity entering the butterfly)
-constexpr int kRowsChunk = 256;   // tokens per staged chunk of a long row = checkpoint spacing of x (kTok * 32)
-
-struct RowsBwdArgs {
-    int batch, dim, L, G, rows_per_group;
-    int softplus;
-    int n_items, nblk, n_chunks;           // nblk: checkpoint slots per half of a chunk; n_chunks: 256-token chunks per row
-    int t0_pct;                            // percent of a chunk's tokens owned by warp 0
-    int tile_bytes, tileo_bytes;            // one [32 x L] tile of u / delta, of dout
-    int off_delta, off_dout, off_bc32, off_ck, off_xch, off_bar, smem_bytes;
-    int Lp;                                 // L rounded up to kBlk (length of the fp32 B' and C rows)
-    const void *u, *delta, *A, *B, *C, *D, *delta_bias, *dout;
-    const float *x;                         // forward checkpoints (batch, dim, n_chunks, 2), read when n_chunks > 1
-    void *du, *ddelta;
-    float *part_dA, *part_dD, *part_dbias, *acc_dB, *acc_dC;
-    long long B_bs, B_gs, C_bs, C_gs;
-};
-
 __device__ __forceinline__ float2 ex2_2(float2 v) { return make_float2(ex2f(v.x), ex2f(v.y)); }
 
 // State of one 16-token block of one row, all in registers (indices are compile-time after unrolling).

@@ -40,26 +40,6 @@
 
 namespace mia {
 
-constexpr int kRnWarps = 4;      // warps per CTA = time slices of a row
-constexpr int kRnBlk = 8;        // tokens per recompute block
-constexpr int kRnOct = 8;        // rows per TMA stage (two quads): 8 L es bytes is a multiple of 16 for every L
-
-struct RowsNBwdArgs {
-    int batch, dim, L, G, rows_per_group;
-    int softplus, has_z;
-    int n_oct, oct_per_cta, oct_per_group;   // work = octets of 8 consecutive rows; CTA c owns [c * oct_per_cta, ...)
-    int nblk, Lp;                            // 8-token blocks per row, nblk * 8
-    int pitch_s, pitch_bc, pitch_acc;        // scratch row pitch (floats), B / C row pitch (elements), accumulator pitch (floats)
-    int max_parts;                           // partial slots per (batch, group) in acc_dB / acc_dC
-    int raw_bytes;                           // one raw tensor tile of 8 rows (in / out dtype sized separately below)
-    int off_raw_u, off_raw_d, off_raw_o, off_raw_z, off_raw_os;   // raw tiles (u, delta, dout, z, out_saved)
-    int off_sm, off_su, off_sy, off_b, off_c, off_acc, off_ck, off_ckm, off_x, off_bar, smem_bytes;
-    const void *u, *delta, *A, *B, *C, *D, *delta_bias, *dout, *z, *out_saved;
-    void *du, *ddelta, *dz;
-    float *part_dA, *part_dD, *part_dbias, *acc_dB, *acc_dC;
-    long long A_ds, A_ns, B_bs, B_gs, B_ns, C_bs, C_gs, C_ns;
-};
-
 // ---- 8 consecutive tokens of two state rows (shared memory, element type T) -> 8 float2 packed over the two states
 template <typename T> struct PairRow;
 template <> struct PairRow<__nv_bfloat16> {

@@ -15,50 +15,12 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "scan_args.h"
+
 namespace mia {
 
-constexpr int kTok = 8;  // tokens per lane per chunk
 constexpr float kLog2e = 1.4426950408889634f;
 constexpr float kLn2 = 0.6931471805599453f;
-constexpr int kMaxStages = 8;
-constexpr int kGroupStages = 2;
-constexpr int kThreads = 512;     // bwd: 15 consumer warps + 1 producer: 4 warps per SM sub-partition, 128 registers each
-constexpr int kThreadsFwd = 512;
-
-// ------------------------------------------------------------------------------------------------
-// Kernel argument block (built on the host by scan_api.cu).
-struct ScanArgs {
-    // problem
-    int batch, dim, L, N, G, delta_dim;
-    int rows_per_group, delta_ratio;
-    int softplus, has_z, out_f32;      // out_f32: dtype of out/out_z (fwd) or dout/out_saved (bwd) is float
-    // tiling
-    int RT, RS, split, tiles_per_seg, LPR, CH, n_chunks, n_seg, stages, n_consumer_warps;
-    // span-merge flags (the rows of a tile are back to back in global memory -> one TMA span)
-    int flat_u, flat_delta, flat_z, flat_dout, flat_osaved, flat_B, flat_C;
-    // shared-memory layout (bytes)
-    int row_pitch, rowo_pitch, bc_pitch;
-    int off_u, off_delta, off_z, off_dout, off_osaved, off_h0, stage_bytes;   // inside a row stage
-    int goff_B, goff_C, goff_A, goff_D, goff_bias, gstage_bytes;              // inside a group stage
-    int off_groups, off_bars, off_carry, off_red, off_bcf, smem_bytes;        // row stages start at 0; off_bcf: fp32 B/C chunk
-                                                                              // of the d_state > 1 fast backward (0 = absent)
-    // pointers
-    const void *u, *delta, *A, *B, *C, *D, *delta_bias, *z;
-    void *out, *out_z;
-    float *x;
-    const void *dout, *out_saved;
-    void *du, *ddelta, *dz;
-    float *part_dA, *part_dD, *part_dbias;   // (batch, dim, N) / (batch, dim) / (batch, dim) f32 partials
-    float *acc_dB, *acc_dC;                  // d_state 1: (parts, N, L) partials ; warp-scan kernels with d_state > 1: (batch, G, N, Lp) red.add accumulators
-    float *ddelta_full;                      // (batch, dim, L) f32 when delta_ratio > 1
-    int bc_atomic;
-    // strides (elements)
-    long long u_bs, u_ds, delta_bs, delta_ds, z_bs, z_ds, A_ds, A_ns;
-    long long B_bs, B_gs, B_ns, C_bs, C_gs, C_ns;
-    long long out_bs, out_ds, outz_bs, outz_ds;
-    long long dout_bs, dout_ds, osaved_bs, osaved_ds;
-    long long du_bs, du_ds, dd_bs, dd_ds, dz_bs, dz_ds;
-};
 
 // ------------------------------------------------------------------------------------------------
 // PTX wrappers: mbarrier, TMA bulk copy, fast math.

@@ -19,19 +19,6 @@
 
 namespace mia {
 
-constexpr int kChunkTok = 256;
-
-struct ChunkArgs {
-    int batch, dim, L, G, rows_per_group;
-    int softplus;
-    int n_chunks, n_items;                 // items = 32-row batches x chunks
-    int tile_bytes, off_bc32, off_bar, smem_bytes;
-    const void *u, *delta, *A, *B, *C, *D, *delta_bias;
-    void *out;
-    float *x;
-    long long B_bs, B_gs, C_bs, C_gs;
-};
-
 template <typename T, bool kSoftplus, bool kOutF32, bool kStateOnly>
 __global__ void __launch_bounds__(32) ss_fwd_chunk_kernel(const __grid_constant__ ChunkArgs a) {
     extern __shared__ __align__(128) char smem[];

@@ -35,22 +35,9 @@
 
 namespace mia {
 
-constexpr int kCwTok = 32;       // columns per window
 #ifndef MIA_CW_OCT
 #define MIA_CW_OCT 1             // 0: the 8-byte (quad) tile accesses of the first version, kept for A/B timing (tools/ab_cw.py)
 #endif
-
-struct CwFwdArgs {
-    int batch, dim, L, G, rows_per_group;
-    int softplus;
-    int g, n_items, nwin, ngrp, ns;         // rows per tensor-map row; items of 32 g rows; windows / 16-column groups per tensor-map row; stages
-    int stage_bytes, off_out, off_bc32, off_bar, smem_bytes;
-    int xchunks, xchunk_tokens;             // checkpoint geometry of x (xchunk_tokens is a power of two >= 32)
-    const void *A, *B, *C, *D, *delta_bias;
-    float *x, *hblk;
-    long long B_bs, B_gs, C_bs, C_gs;
-    int zero;                               // always 0 (the planner zero-fills the block); see `settle` in the kernel
-};
 
 // Per-lane view of its row inside a [32 rows][RB bytes] tile written by TMA (tile base 1024-byte aligned) with the swizzle whose
 // span equals the row: RB = 64 -> CU_TENSOR_MAP_SWIZZLE_64B (16-byte chunk index ^= address bits 7-8), RB = 128 -> SWIZZLE_128B

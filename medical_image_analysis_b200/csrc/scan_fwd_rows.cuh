@@ -20,19 +20,6 @@
 
 namespace mia {
 
-struct RowsArgs {
-    int batch, dim, L, G, rows_per_group;
-    int softplus;
-    int Lc, n_lchunks, n_items;          // tokens per staged chunk, chunks per row, (batch, group, 32-row batch) items
-    int tile_bytes, bc_bytes, off_bc32, stage_bytes, smem_bytes;   // bc_bytes: one raw B (or C) chunk slot incl. alignment
-                                                                   // slack; off_bc32: fp32 copies (B ln2, then C), Lc floats each
-    int xchunks, xchunk_tokens;          // checkpoint geometry of x (shared with the warp-scan kernels)
-    const void *u, *delta, *A, *B, *C, *D, *delta_bias;
-    void *out;
-    float *x;
-    long long B_bs, B_gs, C_bs, C_gs;    // element strides of B / C (sequence stride is 1, d_state == 1)
-};
-
 __device__ __forceinline__ void bulk_s2g(void *gdst, const void *ssrc, uint32_t bytes) {
     asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gdst), "r"(smem_u32(ssrc)), "r"(bytes) : "memory");
 }

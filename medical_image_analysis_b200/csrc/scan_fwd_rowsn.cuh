@@ -23,20 +23,6 @@
 
 namespace mia {
 
-constexpr int kRowsNWarps = 4;   // max warps per CTA: each owns a 32-row batch, all share the B / C rows of the (batch, group)
-
-struct RowsNArgs {
-    int batch, dim, L, G, rows_per_group, N;
-    int softplus;
-    int n_units, units_per_group;         // unit = `warps` consecutive 32-row batches of one (batch, group)
-    int warps, tiles_per_warp;            // 4 warps x (u, delta) tiles, or 2 warps x (u, delta, z) with the z gate
-    int tile_bytes, off_bc, off_bar, smem_bytes;
-    const void *u, *delta, *A, *B, *C, *D, *delta_bias, *z;
-    void *out, *out_z;                    // out_z = out * silu(z) (mamba_ssm signature), both written when z is given
-    float *x;                             // (batch, dim, 1, 2 N): (prod a_n, h_n) at the row end
-    long long A_ds, A_ns, B_bs, B_gs, B_ns, C_bs, C_gs, C_ns;
-};
-
 // kN states of one token, stored as T in shared memory (token-major), to kN/2 float2 state pairs.
 template <typename T, int kN> struct StateRow;
 template <int kN> struct StateRow<__nv_bfloat16, kN> {

@@ -21,20 +21,6 @@
 
 namespace mia {
 
-constexpr int kStreamTok = 32;   // tokens per stage
-
-struct StreamArgs {
-    int batch, dim, L, G, rows_per_group;
-    int softplus;
-    int n_items, Lp;                      // Lp: length of the fp32 B' / C rows
-    int off_bc32, smem_bytes;
-    int xchunks;
-    const void *u, *delta, *A, *B, *C, *D, *delta_bias;
-    void *out;
-    float *x;
-    long long B_bs, B_gs, C_bs, C_gs;
-};
-
 template <int kBytes> __device__ __forceinline__ void cp_async(void *sdst, const void *gsrc) {
     if (kBytes == 16) asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_u32(sdst)), "l"(gsrc) : "memory");
     else asm volatile("cp.async.ca.shared.global [%0], [%1], %2;" ::"r"(smem_u32(sdst)), "l"(gsrc), "n"(kBytes) : "memory");

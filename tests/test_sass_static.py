@@ -49,6 +49,15 @@ def test_forward_does_not_wait_for_its_own_prefetch(g):
 
 
 @needs_objects
+def test_planner_object_compiles_no_scan_kernel():
+    """scan_api.cu reaches the kernels only through the launchers in scan_args.h: its object holds the finalize kernel (one
+    per dtype) and no second copy of a kernel that the per-dtype objects instantiate."""
+    out = subprocess.run(["cuobjdump", "-sass", os.path.join(BUILD, "scan_api.o")], capture_output=True, text=True, check=True).stdout
+    kernels = [l.split("Function :", 1)[1].strip() for l in out.splitlines() if "Function :" in l]
+    assert len(kernels) == 3 and all("ss_finalize_kernel" in k for k in kernels), kernels
+
+
+@needs_objects
 def test_blackwell_instructions_present():
     def count(obj, needle):
         out = subprocess.run(["cuobjdump", "-sass", os.path.join(BUILD, obj)], capture_output=True, text=True, check=True).stdout
